@@ -2,6 +2,7 @@
 """bench.py -- pod-fit decisions/s of the autoscaler tick on B200 (driver contract, see DESIGN.md section 6).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c3|small]
+                    [--dump-outputs DIR]
 
 A "step" is one whole tick of the hot path over one synthetic snapshot (SURVEY.md section 8d):
     occupancy (K1) + get_pods_to_schedule (K0) + get_pending_pods (first-fit pipeline over nodes)
@@ -18,6 +19,9 @@ N > 1 (torchrun, one rank per GPU): ONE cluster -- c3 -- on all ranks in cluster
 scaling; the result is asserted equal, bit for bit, to the single-GPU result of the same snapshot computed in the
 same run, whose time is reported next to it (`strong_scaling`).  `configs.c4` (10M x 1M, N = 8) and the former
 weak-scaling "fleet" measurement are secondary keys.
+
+--dump-outputs DIR writes what the last timed step of the headline tick returned, as DIR/<name>.npy in float64
+(see dump_outputs), so that two builds can be compared output for output on the same seeded snapshot.
 """
 import argparse
 import json
@@ -44,6 +48,8 @@ C5_THRESHOLDS = [60, 300, 900, 1800, 3600, 7200, 21600, 86400]
 METRIC = "pod-fit decisions/sec"
 UNIT = "decisions/s"
 SEED = 20260921 + 2
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SAMPLE_SEED = 20260921
 
 
 def load_peaks():
@@ -228,7 +234,7 @@ def run_reference(args):
     from kubernetes_acs_engine_autoscaler_b200 import synthetic as syn
     name = args.config if args.gpus == 1 else "c3"
     P, N, D, T = CONFIGS[name]
-    steps, warmup = max(1, min(args.steps, 4)), min(args.warmup, 1)
+    steps, warmup = args.steps, args.warmup
     # the C port on a bounded sample of the same workload (full c2; c3 scaled to 1/8 of the pods and nodes)
     Ps, Ns = (P, N) if P * N <= 2 * 10 ** 9 else (P // 8, N // 8)
     cs = syn.make_cluster(Ps, Ns, D, T, seed=SEED)
@@ -324,8 +330,17 @@ class Workload(object):
         r = eng.scale_up(d["req"], *self.pool_args(), d["cap_type"], d["node_type"], self.used)  # rows F0, F1, F
         st = eng.node_states(d["row_ptr"], d["run_idx"], d["req_run"], d["flags_run"], d["cap_type"], d["node_type"],
                              d["node_flags"], d["node_age"], r["n_to_schedule"] > 0, self.thr)   # row I (K6)
-        eng.maintain_actions(st[0], d["node_pool"], self.budget, self.scalable, True)            # row J
+        self.last_maintain = eng.maintain_actions(st[0], d["node_pool"], self.budget, self.scalable, True)  # row J
         return r
+
+    def outputs(self, r):
+        """what a caller of step_device receives from the step that returned `r` (host copies)."""
+        state, action = self.last_maintain
+        out = {k: r[k].cpu().numpy() for k in ("feasible", "placed", "acc_pool")}
+        out.update({k: r[k] for k in ("new_size", "units_needed", "bins_opened")})
+        out.update({k: np.array([r[k]]) for k in ("n_to_schedule", "n_pending", "num_unaccounted", "decisions")})
+        out.update({"used": self.used.cpu().numpy(), "node_state": state.cpu().numpy(), "node_action": action.cpu().numpy()})
+        return out
 
     def step_host(self):
         eng, h = self.eng, self.h
@@ -355,6 +370,27 @@ class Workload(object):
             byt += algorithmic_bytes(s["decisions"], c["P"], c["N"] + int(r["bins_opened"].sum()), c["D"])
         eng.set_timing(False)
         return ms / reps, dec / reps, byt / reps
+
+
+def dump_outputs(directory, arrays):
+    """write each array as <directory>/<name>.npy in float64 (exact for the int32 / int64 counts and uint8 codes
+    the tick returns).  Should the whole exceed DUMP_LIMIT_BYTES, arrays are cut along their first axis to one fixed,
+    seeded sample of rows (the same rows for every array of the same length), and the row numbers are written as
+    <name>_rows.npy.  Arrays of at most 65536 rows (pool sizes, counts) are always written whole."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    big = [k for k, a in arrays.items() if a.ndim and a.shape[0] > 65536]
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        small = total - sum(arrays[k].nbytes for k in big)
+        keep = (DUMP_LIMIT_BYTES - small) / (2.0 * (total - small))  # half of what is left: room for the row numbers
+        for name in big:
+            a = arrays[name]
+            rows = np.sort(np.random.default_rng(DUMP_SAMPLE_SEED).choice(a.shape[0], int(a.shape[0] * keep), replace=False))
+            arrays[name], arrays[name + "_rows"] = a[rows], rows.astype(np.float64)
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_LIMIT_BYTES
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 LAST_STEP_MS = []
@@ -565,6 +601,8 @@ def run_single(args):
     with ClockSampler(0) as clocks:
         res, dev_ms, launches = timed(w.step_device, args.steps, args.warmup, flush, nb, lambda: eng.launch_count, MIN_WARM_SECONDS)
         step_ms, steps_in_order = sorted(LAST_STEP_MS), [round(x, 3) for x in LAST_STEP_MS]
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, w.outputs(res))
         res_h, host_ms, _ = timed(w.step_host, args.steps, max(1, args.warmup // 2), flush, nb, lambda: eng.launch_count, MIN_WARM_SECONDS)
     assert res_h["decisions"] == res["decisions"]
     k_ms, k_dec, k_bytes = w.pipeline_leg(flush, max(1, min(args.steps, 5)))
@@ -670,7 +708,7 @@ def run_cluster(args):
         t = t.cpu().numpy()
         assert np.array_equal(t[:len(v)], v) and np.array_equal(-t[len(v):], v), "ranks disagree on the pool counts"
 
-    def measure(cname, steps, warmup, verify=True, solo_steps=2):
+    def measure(cname, steps, warmup, verify=True, solo_steps=2, dump_dir=None):
         Pc, Nc, Dc, Tc = CONFIGS[cname]
         c = syn.make_cluster(Pc, Nc, Dc, Tc, seed=SEED)  # identical on every rank
         w = Workload(eng, c, pinned=(cname != "c4"))
@@ -680,6 +718,8 @@ def run_cluster(args):
             counts_agree(r, c)
             return r
         res, dev_ms, launches = timed(step, steps, warmup, flush, barrier, lambda: eng.launch_count)
+        if dump_dir and rank == 0:  # every rank holds the whole (replicated) result
+            dump_outputs(dump_dir, w.outputs(res))
         plan = eng.cluster_last_plan()
         host_ms = None
         if w.h is not None:
@@ -743,7 +783,7 @@ def run_cluster(args):
         return rec, c
 
     with ClockSampler(local_rank) as clocks:
-        head, c = measure(name, args.steps, args.warmup)
+        head, c = measure(name, args.steps, args.warmup, dump_dir=args.dump_outputs)
     line = {
         "metric": METRIC, "value": head["value"], "unit": UNIT, "n_gpus": world, "steps": args.steps,
         "warmup": args.warmup, "ms_per_step": head["ms_per_step"], "higher_is_better": True, "scaling": "strong",
@@ -804,7 +844,13 @@ def main():
     ap.add_argument("--no-c4", action="store_true", help="N > 1: skip the configs.c4 sub-record (10M x 1M, ~1 minute)")
     ap.add_argument("--no-c4-verify", action="store_true", help="skip the single-GPU check of c4 (tens of seconds)")
     ap.add_argument("--no-fleet", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup not negative")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU tick (--impl ours)")
+    sys.dont_write_bytecode = True  # the tree may be read-only: nothing imported from here leaves a cache in it
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":
         run_reference(args)

@@ -1,7 +1,8 @@
-"""`-m "not gpu"`, only where the reference is present: the HOST LAYER of this package (Cluster.loop_logic: object
-construction incl. the C helper, flattening, hand-off, write-back of `used_capacity`, maintain) on mid-size synthetic
-clusters against the unmodified reference run live on the same kube-style objects.  The device work is done by the
-plain-C oracle here (tests/oracle_engine.py); the CUDA engine behind the same layer is checked by the GPU suite."""
+"""`-m "not gpu"`: the HOST LAYER of this package (Cluster.loop_logic: object construction incl. the C helper,
+flattening, hand-off, write-back of `used_capacity`, maintain) on mid-size synthetic clusters against the unmodified
+reference run on the same kube-style objects, as recorded in tests/golden/live_ticks.json.gz
+(oracle/make_golden_live.py).  The device work is done by the plain-C oracle here (tests/oracle_engine.py); the CUDA
+engine behind the same layer is checked by the GPU suite."""
 import logging
 import os
 import re
@@ -12,9 +13,7 @@ import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(os.path.dirname(HERE), "oracle"))
-import ref_shim  # noqa: E402
-
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present")
+import live_golden  # noqa: E402
 
 
 class Raw(object):
@@ -46,14 +45,17 @@ def test_loop_logic_equals_the_live_reference(oracle_mod, tmp_path, monkeypatch,
     from kubernetes_acs_engine_autoscaler_b200 import synthetic as syn
     from kubernetes_acs_engine_autoscaler_b200.cluster import Cluster
 
-    c = syn.make_cluster(P, N, D, T, seed=seed, over_provision=1)
+    rec = live_golden.find("host_layer", P=P, N=N, D=D, T=T, seed=seed, max_size=max_size)
+    c = live_golden.cluster_of(rec)
+    assert c["over_provision"] == 1
     cap = int(max_size if max_size is not None else c["pool_max"][0])
 
-    # ---- the reference, live -------------------------------------------------------------------
-    tick = ref_bench.ReferenceTick(c, tmpdir=str(tmp_path), max_size=cap)
-    ref = tick.run(record=True)
-    ref_keys = [set(n.used_capacity.raw) for n in tick.nodes]
-    ref_state = {n.name: s for n, s in zip(tick.nodes, ref["states"])}
+    # ---- the reference, as recorded on the same objects ------------------------------------------
+    ref = live_golden.tick_result(rec)
+    ref_names = rec["node_names"]
+    ref_keys = live_golden.key_sets(live_golden._unpack(rec["used_keys"], np.uint8), c["dim_names"])
+    ref_state = {name: live_golden.STATE_NAMES[int(s)]
+                 for name, s in zip(ref_names, live_golden._unpack(rec["states"], np.uint8))}
 
     # ---- this package's host layer on the same objects -----------------------------------------
     st = syn.kube_objects(c)
@@ -80,7 +82,7 @@ def test_loop_logic_equals_the_live_reference(oracle_mod, tmp_path, monkeypatch,
     monkeypatch.setattr(utils, "now", lambda tz=None: syn.NOW if tz is None else syn.NOW.astimezone(tz))
     prev = snapshot._engine
     snapshot.set_engine(OracleEngine())
-    capacity.load(ref_bench.capacity_file(c, str(tmp_path)))  # the table the reference run above was given (D = 8: generated)
+    capacity.load(ref_bench.capacity_file(c, str(tmp_path)))  # the table the reference was given (D = 8: generated)
     handler = Lines()
     log = logging.getLogger("autoscaler")
     log.addHandler(handler)
@@ -104,7 +106,7 @@ def test_loop_logic_equals_the_live_reference(oracle_mod, tmp_path, monkeypatch,
         assert exc[0] == ref["exception"][0]
     assert scale_calls == ref["scale_calls"]
     names = c["dim_names"]
-    assert [n.name for n in kube_nodes] == [n.name for n in tick.nodes]
+    assert [n.name for n in kube_nodes] == ref_names
     used = np.array([[float(n.used_capacity.raw.get(k, 0.0)) for k in names] for n in kube_nodes], dtype=np.float64)
     assert np.array_equal(used.view(np.uint64), ref["used"].view(np.uint64))
     assert [set(n.used_capacity.raw) for n in kube_nodes] == ref_keys      # KubeResource.__add__ unions the key sets
@@ -118,4 +120,4 @@ def test_loop_logic_equals_the_live_reference(oracle_mod, tmp_path, monkeypatch,
             if m:
                 got_state[re.search(r"(k8s-[a-z0-9]+-\d+-\d+)", m.group(1)).group(1)] = m.group(2)
         assert len(got_state) == len(kube_nodes)
-        assert got_state == {k: str(v) for k, v in ref_state.items()}
+        assert got_state == ref_state

@@ -1,20 +1,18 @@
 """ARM template unrolling (SURVEY.md section 8(f)3): the reference's own known-answer tests
-(test/test_template_processing.py:34-89) and, where the reference is present, a differential run of every
-function on the reference's fixture templates."""
+(test/test_template_processing.py:34-89) and a differential run of every function on the reference's fixture
+templates.  The fixtures and what the unmodified reference returned on them are recorded in
+tests/golden/template_fixtures.json.xz (oracle/make_golden_live.py)."""
 import copy
 import json
+import lzma
 import os
-import sys
 
 import pytest
 
 from kubernetes_acs_engine_autoscaler_b200 import template_processing as tp
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-sys.path.insert(0, os.path.join(os.path.dirname(HERE), "oracle"))
-import ref_shim  # noqa: E402
-
-REF_DATA = os.path.join(ref_shim.REFERENCE_ROOT, "test", "data")
+FIXTURES = os.path.join(HERE, "golden", "template_fixtures.json.xz")
 
 
 class Node(object):
@@ -94,38 +92,36 @@ def test_scale_out_template_shape():
     assert len(tp.delete_master_vm_extension(mini_template())["resources"]) == len(mini_template()["resources"]) - 1
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_DATA) or not ref_shim.available(), reason="reference fixtures not present")
-def test_every_function_equals_the_reference_on_its_fixtures():
-    ns = ref_shim.load_reference()
-    import importlib
-    sys.path.insert(0, ref_shim.REFERENCE_ROOT)
-    try:
-        ref_tp = importlib.import_module("autoscaler.template_processing")
-    finally:
-        sys.path.remove(ref_shim.REFERENCE_ROOT)
-    del ns
-
-    def load(name):
-        with open(os.path.join(REF_DATA, name)) as f:
-            return json.load(f)
-    original = load("azuredeploy.original.json")
-    pool = Pool("agentpool1", [0])
-    # the reference's two fixture KATs (test/test_template_processing.py:34-56)
-    assert tp.unroll_nic(copy.deepcopy(original), pool, 3) == load("azuredeploy.expected_nic.json")
-    assert tp.unroll_vm(copy.deepcopy(original), pool, 3) == load("azuredeploy.expected_vm.json")
-    cluster = load("azuredeploy.cluster.json")
+def differential_calls(cluster):
+    """the calls compared with the reference on its cluster fixture: key -> (function name, fresh arguments)."""
     pool_names = sorted({r["name"].split("variables('")[1].split("VMNamePrefix")[0] for r in cluster["resources"]
                          if "VMNamePrefix'), copyIndex" in r["name"] and "master" not in r["name"]})
     assert pool_names
-    for sizes, held in [({n: 3 for n in pool_names}, [0]), ({n: 1 for n in pool_names}, [0]),
-                        ({n: (5 if i == 0 else 2) for i, n in enumerate(pool_names)}, [1, 3])]:
-        pools = [Pool(n, held) for n in pool_names]
-        assert tp.prepare_template_for_scale_out(copy.deepcopy(cluster), pools, dict(sizes)) == \
-            ref_tp.prepare_template_for_scale_out(copy.deepcopy(cluster), pools, dict(sizes))
+    calls = {}
+    for k, (sizes, held) in enumerate([({n: 3 for n in pool_names}, [0]), ({n: 1 for n in pool_names}, [0]),
+                                       ({n: (5 if i == 0 else 2) for i, n in enumerate(pool_names)}, [1, 3])]):
+        calls["prepare_template_for_scale_out/%d" % k] = (
+            "prepare_template_for_scale_out",
+            lambda sizes=sizes, held=held: (copy.deepcopy(cluster), [Pool(n, held) for n in pool_names], dict(sizes)))
     for fn in ("unroll_vm_extension", "unroll_nic", "unroll_vm"):
-        assert getattr(tp, fn)(copy.deepcopy(cluster), Pool(pool_names[0], [0, 2]), 5) == \
-            getattr(ref_tp, fn)(copy.deepcopy(cluster), Pool(pool_names[0], [0, 2]), 5)
-    assert tp.delete_master_vm_extension(copy.deepcopy(cluster)) == ref_tp.delete_master_vm_extension(copy.deepcopy(cluster))
-    assert tp.delete_nsg(cluster) == ref_tp.delete_nsg(cluster)
-    assert tp.delete_unchanged_pools(copy.deepcopy(cluster), [Pool(pool_names[0], [0])]) == \
-        ref_tp.delete_unchanged_pools(copy.deepcopy(cluster), [Pool(pool_names[0], [0])])
+        calls[fn] = (fn, lambda: (copy.deepcopy(cluster), Pool(pool_names[0], [0, 2]), 5))
+    for fn in ("delete_master_vm_extension", "delete_nsg"):
+        calls[fn] = (fn, lambda: (copy.deepcopy(cluster),))
+    calls["delete_unchanged_pools"] = ("delete_unchanged_pools",
+                                       lambda: (copy.deepcopy(cluster), [Pool(pool_names[0], [0])]))
+    return calls
+
+
+def test_every_function_equals_the_reference_on_its_fixtures():
+    with lzma.open(FIXTURES, "rb") as f:
+        golden = json.loads(f.read().decode())
+    fixtures = golden["fixtures"]
+    original = fixtures["azuredeploy.original.json"]
+    pool = Pool("agentpool1", [0])
+    # the reference's two fixture KATs (test/test_template_processing.py:34-56)
+    assert tp.unroll_nic(copy.deepcopy(original), pool, 3) == fixtures["azuredeploy.expected_nic.json"]
+    assert tp.unroll_vm(copy.deepcopy(original), pool, 3) == fixtures["azuredeploy.expected_vm.json"]
+    calls = differential_calls(fixtures["azuredeploy.cluster.json"])
+    assert sorted(calls) == sorted(golden["results"])
+    for key, (fn, args) in calls.items():
+        assert getattr(tp, fn)(*args()) == golden["results"][key], key
